@@ -22,8 +22,12 @@ owns its own 4096 voices; the only data-path collective is the mix-bus sum (SURV
            mix bus are compared with the reference engine advanced by exactly as many blocks (parity_checked,
            worst_err_over_tol).  A bench line whose kernel computed something else says so.
   cpu_baseline / --impl reference: the UNMODIFIED reference engine (oracle/_ref/libelem_ref.so, built from
-           /root/reference in place) on the box's host cores: T = all threads (value) and T = 1, pinned threads created
+           the reference sources in place) on the box's host cores: T = all threads (value) and T = 1, pinned threads created
            and warmed up outside the timed region, >= 2 s timed (oracle/ref_driver.cpp:elem_ref_bench_stable).
+  --dump-outputs DIR: after the timed steps, the mix bus [1][512] (float32) that the last step of the `value` loop left in the
+           engine — what enqueue_block hands its caller — as DIR/mix.npy, and that of the 131072-voice row as DIR/t1_mix.npy.
+           Every input is fixed by the arguments (per-voice f0 from the voice index, no random state), so two builds of the
+           project run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -231,7 +235,7 @@ def class_references(n_blocks):
     return out, cls.__name__
 
 
-def measure(args, voices, steps, warmup, rank, local_rank, world, stream, flush, with_clocks, check_parity):
+def measure(args, voices, steps, warmup, rank, local_rank, world, stream, flush, with_clocks, check_parity, keep_mix=False):
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -310,6 +314,7 @@ def measure(args, voices, steps, warmup, rank, local_rank, world, stream, flush,
     barrier()
     t_wall = time.perf_counter() - t_wall0
     dev_ms = sum(a.elapsed_time(b) for a, b in evs)
+    last_mix = mix.cpu().numpy().copy() if keep_mix else None      # the last timed step's output, before the passes below overwrite it
     launches = rt.kernel_launches - launches0      # K1 + K2 (+ K4) per step; the line-up barriers are not counted by the engine
 
     # ---- per-kernel durations (roofline, kernel_ms): the same steps once more, event pairs around every launch ----
@@ -381,7 +386,7 @@ def measure(args, voices, steps, warmup, rank, local_rank, world, stream, flush,
     res = {"voices": voices, "steps": steps, "dev_ms": float(t[0]), "e2e_ms": float(t[1]), "k1_ms": float(t[2]), "k1_n": k1_n,
            "k2_ms": float(t[3]), "k2_n": kinds["K2"][1], "k4_ms": float(t[4]), "k4_n": kinds["K4"][1],
            "launches": int(launches), "t_wall": t_wall, "clocks": clocks, "desc": desc, "fused": fused, "fused_note": fused_note,
-           "peer_fail": peer_fail, "parity": parity}
+           "peer_fail": peer_fail, "parity": parity, "last_mix": last_mix}
     rt.close()
     return res
 
@@ -402,15 +407,22 @@ def run_b200(args, rank, local_rank, world, emit=print):
     stream = torch.cuda.Stream()
     with torch.cuda.stream(stream):
         flush = torch.empty(256 << 20, dtype=torch.uint8, device=f"cuda:{local_rank}")
-        m = measure(args, voices, args.steps, args.warmup, rank, local_rank, world, stream, flush, True, not args.no_parity)
+        keep = bool(args.dump_outputs)
+        m = measure(args, voices, args.steps, args.warmup, rank, local_rank, world, stream, flush, True, not args.no_parity, keep)
         t1 = None
         if not args.no_t1 and voices != T1_VOICES_PER_GPU:      # row T1: the 1 M-voice target = 131072 voices on each of 8 GPUs
-            t1 = measure(args, T1_VOICES_PER_GPU, min(args.steps, 30), 5, rank, local_rank, world, stream, flush, False, not args.no_parity)
+            t1 = measure(args, T1_VOICES_PER_GPU, min(args.steps, 30), 5, rank, local_rank, world, stream, flush, False, not args.no_parity, keep)
         if world > 1:
             dist.barrier()
             dist.destroy_process_group()
     if rank != 0:
         return
+    if args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "mix.npy"), m["last_mix"].astype(np.float32))
+        if t1 is not None:
+            np.save(os.path.join(args.dump_outputs, "t1_mix.npy"), t1["last_mix"].astype(np.float32))
 
     steps = args.steps
     dev_ms, e2e_ms = m["dev_ms"], m["e2e_ms"]
@@ -540,7 +552,13 @@ def main():
     ap.add_argument("--collective", default="fused", choices=["fused", "nccl"], help="N > 1: K4 peer-memory kernel (default) or NCCL all_reduce")
     ap.add_argument("--tile-width", type=int, default=0, help="override the voices-per-warp heuristic (exploration only)")
     ap.add_argument("--opt", action="append", default=[], help="extra runtime option key=value (exploration only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the mix bus of the last timed step as DIR/mix.npy (and DIR/t1_mix.npy), see the module docstring")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200: the reference arm reports a checksum, not the rendered samples")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -133,3 +133,24 @@ def case_inputs(case, bs=512, seed=0):
     if not case["n_in"]:
         return None
     return np.stack([lcg_noise(case["n_blocks"] * bs, seed * 100 + c) for c in range(case["n_in"])])
+
+
+def convolve_rounding_render(cls, taps, sr=48000.0, bs=512):
+    """36 blocks of noise through the convolver on the first `taps` taps of the config-4 IR: [1, 36 * bs]."""
+    ir = np.asarray(graphs.lcg_ir(16384)[:taps], dtype=np.float32)
+    rng = np.random.RandomState(3)
+    x = ((rng.rand(1, 36 * bs) - 0.5) * 0.5).astype(np.float32)
+    r = cls(sr, bs)
+    assert r.add_shared_resource("ir", ir) and r.apply(graphs.convolve_channel("ir")) == 0
+    return r.render(36, 1, bs, x)
+
+
+def plugin_nodes_batch():
+    """The graph of the registered-node-type test: 3 * in0 -> softclip -> leaky (g = 0.9), plus 0.1 * cycle(330)."""
+    soft = el.create_node("b200test.softclip", {}, [el.mul(3.0, IN0)])
+    return el.render(el.add(el.create_node("b200test.leaky", {}, [soft, el.const(0.9, key="g")]), el.mul(0.1, el.cycle(330.0))))
+
+
+def plugin_nodes_inputs(n_voices, bs=512):
+    """[voice, 1, 4 * bs]: 4 blocks of LCG noise per voice."""
+    return np.stack([np.stack([lcg_noise(4 * bs, 100 * v)]) for v in range(n_voices)])

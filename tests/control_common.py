@@ -1,5 +1,7 @@
 """Live-update scenarios for the sequencing / control nodes, shared by the GPU parity tests (CUDA path vs oracle) and the CPU
 pinning test (restatement vs compiled reference): an initial batch plus batches applied before given blocks."""
+import numpy as np
+
 from elementary_b200 import el
 
 TRIG = el.train(2000.0)
@@ -50,3 +52,22 @@ def scenarios():
         4: [[3, dly.id(), "size", 600]],
         5: [[3, svf.id(), "mode", "notch"]]}))
     return out
+
+
+def definition(sc):
+    """What a scenario renders, as JSON-able data (the stored reference outputs are tied to it by digest)."""
+    return {k: sc.get(k) for k in ("batch", "n_blocks", "n_out", "sample_times")} | {"script": {str(b): v for b, v in sc["script"].items()}}
+
+
+def render_live(cls, sc, sr=48000.0, bs=512):
+    """A scenario on an oracle class: the script's batches applied before their blocks, [n_out, n_blocks * bs]."""
+    r = cls(sr, bs)
+    assert r.apply(sc["batch"]) == 0
+    blocks = []
+    for b in range(sc["n_blocks"]):
+        if b in sc["script"]:
+            assert r.apply(sc["script"][b]) == 0
+        if sc.get("sample_times"):
+            r.set_current_time(sc["sample_times"][b])
+        blocks.append(r.process(None, sc["n_out"], bs))
+    return np.concatenate(blocks, axis=1)

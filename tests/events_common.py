@@ -34,6 +34,19 @@ def scenarios():
     ]
 
 
+def event_log(cls, sc, sr=48000.0, bs=512):
+    """[(block, canonical events)] of one scenario on an oracle class, polled on the scenario's schedule."""
+    r = cls(sr, bs)
+    assert r.apply(el.render(*sc["graph"])) == 0
+    log = []
+    for b in range(sc["blocks"]):
+        x = np.stack([noise(bs, 1000 * b + c) for c in range(sc["n_in"])]) if sc["n_in"] else None
+        r.process(x, len(sc["graph"]), bs)
+        if sc["poll"](b):
+            log.append((b, canon(r.process_queued_events())))
+    return log
+
+
 def noise(n, seed):
     rng = np.random.RandomState(seed)
     return (rng.rand(n).astype(np.float32) * 2.0 - 1.0)
@@ -74,5 +87,46 @@ def same(got, want):
             a, b = np.asarray(eg["data"][part], dtype=np.float64), np.asarray(ew["data"][part], dtype=np.float64)
             scale = max(1e-30, np.abs(np.asarray(ew["data"]["real"])).max(), np.abs(np.asarray(ew["data"]["imag"])).max())
             if a.shape != b.shape or np.abs(a - b).max() > 2e-6 * scale:
+                return False
+    return True
+
+
+FFT_BINS = 128
+
+
+def fingerprint(events):
+    """Compact stored form of a canonical event list (tests/golden/reference_extra.json): an event that `same` compares exactly
+    is kept as a digest of its content; an `fft` event as its source, length, the peak `same` scales its tolerance by and
+    FFT_BINS bins at fixed positions."""
+    from helpers import sha16
+    out = []
+    for t, e in events:
+        if t != "fft":
+            out.append({"type": t, "sha256_16": sha16(e)})
+            continue
+        re_, im = np.asarray(e["data"]["real"], dtype=np.float64), np.asarray(e["data"]["imag"], dtype=np.float64)
+        bins = np.sort(np.random.RandomState(len(re_)).choice(len(re_), min(FFT_BINS, len(re_)), replace=False))
+        out.append({"type": t, "source": e.get("source"), "n": len(re_), "scale": max(1e-30, np.abs(re_).max(), np.abs(im).max()),
+                    "bins": bins.tolist(), "real": re_[bins].tolist(), "imag": im[bins].tolist()})
+    return out
+
+
+def same_as_fingerprint(got, want):
+    """`same`, with the expected event list in its stored form (`fingerprint`)."""
+    from helpers import sha16
+    if len(got) != len(want):
+        return False
+    for (tg, eg), w in zip(got, want):
+        if tg != w["type"]:
+            return False
+        if tg != "fft":
+            if sha16(eg) != w["sha256_16"]:
+                return False
+            continue
+        if eg.get("source") != w["source"]:
+            return False
+        for part in ("real", "imag"):
+            a = np.asarray(eg["data"][part], dtype=np.float64)
+            if a.shape != (w["n"],) or np.abs(a[w["bins"]] - np.asarray(w[part])).max() > 2e-6 * w["scale"]:
                 return False
     return True

@@ -1,9 +1,28 @@
 """Shared helpers for the parity tests (tests only)."""
 from __future__ import annotations
 
+import hashlib
+import json
+import os
+
 import numpy as np
 
 from oracle import oracle as orc
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def sha16(obj) -> str:
+    """First 16 hex digits of the SHA-256 of ``obj`` as JSON: ties a stored fixture to the definition it was rendered from."""
+    return hashlib.sha256(json.dumps(obj, sort_keys=True).encode()).hexdigest()[:16]
+
+
+def reference_extra():
+    """(arrays, metadata) of tests/golden/reference_extra.{npz,json}: what the reference engine rendered for the tests that
+    compare with it beyond reference_cases (tests/golden/make_ref_fixtures.py)."""
+    with open(os.path.join(GOLDEN, "reference_extra.json")) as f:
+        meta = json.load(f)
+    return np.load(os.path.join(GOLDEN, "reference_extra.npz")), meta
 
 
 def oracle_cls():

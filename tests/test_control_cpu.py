@@ -1,31 +1,22 @@
-"""CPU: the restatement (oracle/elem_oracle.cpp) against the compiled reference on the LIVE-UPDATE scenarios of the sequencing /
+"""CPU: the restatement (oracle/elem_oracle.cpp) against the reference engine on the LIVE-UPDATE scenarios of the sequencing /
 control nodes (tests/control_common.py) — new sequence data, loop points, re-arming, host clock jumps, baked properties changed
 between blocks.  Everything except transcendental-free paths must be bit-exact; the others agree to float rounding of libm-free
-double arithmetic, i.e. exactly as well."""
+double arithmetic, i.e. exactly as well.  The reference's outputs are stored in tests/golden/reference_extra.npz."""
 import numpy as np
 import pytest
 
-from control_common import scenarios
+from control_common import definition, render_live, scenarios
+from helpers import reference_extra, sha16
 from oracle import oracle as orc
 
 SR, BS = 48000.0, 512
 SCEN = scenarios()
+GOLD, META = reference_extra()
 
 
-@pytest.mark.skipif(not orc.ref_available(), reason="oracle/_ref not built (no /root/reference here)")
 @pytest.mark.parametrize("sc", SCEN, ids=[s["name"] for s in SCEN])
 def test_port_matches_reference_through_live_updates(sc):
-    outs = []
-    for cls in (orc.PortRuntime, orc.RefRuntime):
-        r = cls(SR, BS)
-        assert r.apply(sc["batch"]) == 0
-        blocks = []
-        for b in range(sc["n_blocks"]):
-            if b in sc["script"]:
-                assert r.apply(sc["script"][b]) == 0
-            if sc.get("sample_times"):
-                r.set_current_time(sc["sample_times"][b])
-            blocks.append(r.process(None, sc["n_out"], BS))
-        outs.append(np.concatenate(blocks, axis=1))
-    assert np.array_equal(outs[0], outs[1]), f"{sc['name']}: max diff {np.abs(outs[0] - outs[1]).max()}"
-    assert np.abs(outs[1]).max() > 0
+    assert META["sha256_16"]["control_" + sc["name"]] == sha16(definition(sc)), "scenario changed: re-run tests/golden/make_ref_fixtures.py"
+    got, want = render_live(orc.PortRuntime, sc), GOLD["control_" + sc["name"]]
+    assert np.array_equal(got, want), f"{sc['name']}: max diff {np.abs(got - want).max()}"
+    assert np.abs(want).max() > 0

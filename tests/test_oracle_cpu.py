@@ -1,16 +1,20 @@
-"""CPU: pin the oracle.  (1) the restatement (oracle/elem_oracle.cpp) must agree BIT-EXACTLY with the compiled
-reference (oracle/_ref, present wherever /root/reference was available at build time) on every node family;
-(2) both must reproduce the reference's own golden vectors (jest snapshots) and the Appendix-E anchors."""
+"""CPU: pin the oracle.  (1) the restatement (oracle/elem_oracle.cpp) must agree BIT-EXACTLY with the reference engine's
+outputs on every node family (stored under tests/golden/, rendered by the unmodified reference compiled into oracle/_ref);
+(2) the restatement, and the compiled reference where oracle/_ref was built, must reproduce the reference's own golden
+vectors (jest snapshots) and the Appendix-E anchors."""
+import os
+
 import numpy as np
 import pytest
 
 from elementary_b200 import el, graphs
 from oracle import oracle as orc
-from cases import CASES, case_inputs
+from cases import CASES, case_inputs, convolve_rounding_render
+from helpers import GOLDEN, reference_extra, sha16
 
 SR, BS = 48000.0, 512
-
-needs_ref = pytest.mark.skipif(not orc.ref_available(), reason="oracle/_ref not built (no /root/reference here)")
+CASES_GOLD = np.load(os.path.join(GOLDEN, "reference_cases.npz"))
+GOLD, META = reference_extra()
 
 
 def render(cls, case, sr=SR):
@@ -21,11 +25,11 @@ def render(cls, case, sr=SR):
     return r.render(case["n_blocks"], case["n_out"], BS, case_inputs(case))
 
 
-@needs_ref
 @pytest.mark.parametrize("case", CASES, ids=[c["name"] for c in CASES])
 def test_port_matches_compiled_reference_bit_exactly(case):
+    """Against the reference's render of the case, stored in tests/golden/reference_cases.npz (test_golden.py checks it is current)."""
     a = render(orc.PortRuntime, case)
-    b = render(orc.RefRuntime, case)
+    b = CASES_GOLD[case["name"]]
     assert np.array_equal(a, b), f"{case['name']}: max diff {np.abs(a - b).max()}"
 
 
@@ -128,18 +132,12 @@ def test_convolve_against_exact_convolution(cls, taps, blocks):
     assert np.abs(got[2 * BS:] - want[2 * BS:]).max() <= 1e-6 * peak      # after the 20 ms root fade-in
 
 
-@needs_ref
 @pytest.mark.parametrize("taps", [300, 5000, 16384])
 def test_convolve_port_matches_reference_to_float_rounding(taps):
-    ir = np.asarray(graphs.lcg_ir(16384)[:taps], dtype=np.float32)
-    rng = np.random.RandomState(3)
-    x = ((rng.rand(1, 36 * BS) - 0.5) * 0.5).astype(np.float32)
-    outs = []
-    for cls in (orc.PortRuntime, orc.RefRuntime):
-        r = cls(SR, BS)
-        assert r.add_shared_resource("ir", ir) and r.apply(graphs.convolve_channel("ir")) == 0
-        outs.append(r.render(36, 1, BS, x))
-    assert np.abs(outs[0] - outs[1]).max() <= 5e-7 * np.abs(outs[1]).max()
+    """Against the reference's output stored at 2048 fixed positions, with its exact peak (tests/golden/reference_extra.npz)."""
+    got = convolve_rounding_render(orc.PortRuntime, taps)[0]
+    idx = GOLD["convolve_rounding_idx"]
+    assert np.abs(got[idx] - GOLD[f"convolve_rounding_{taps}"]).max() <= 5e-7 * GOLD[f"convolve_rounding_{taps}_peak"]
 
 
 @pytest.mark.parametrize("cls", _checkers(), ids=lambda c: c.__name__)
@@ -158,21 +156,12 @@ def test_convolve_varying_call_lengths_is_still_a_plain_convolution(cls):
 
 
 # ---- events (SURVEY.md §8f N4): the restatement's processQueuedEvents against the compiled reference ----------------
-@needs_ref
 def test_port_events_match_compiled_reference():
-    from events_common import scenarios, noise, canon, same
+    """Against the reference's event logs in their stored form (events_common.fingerprint, tests/golden/reference_extra.json)."""
+    from events_common import event_log, scenarios, same_as_fingerprint
     for sc in scenarios():
-        batch = el.render(*sc["graph"])
-        runs = []
-        for cls in (orc.PortRuntime, orc.RefRuntime):
-            r = cls(SR, BS)
-            assert r.apply(batch) == 0
-            log = []
-            for b in range(sc["blocks"]):
-                x = np.stack([noise(BS, 1000 * b + c) for c in range(sc["n_in"])]) if sc["n_in"] else None
-                r.process(x, len(sc["graph"]), BS)
-                if sc["poll"](b):
-                    log.append((b, canon(r.process_queued_events())))
-            runs.append(log)
-        assert len(runs[0]) == len(runs[1]) and all(b0 == b1 and same(e0, e1) for (b0, e0), (b1, e1) in zip(*runs)), sc["name"]
-        assert any(ev for _, ev in runs[1]) != bool(sc.get("silent")), sc["name"] + ": unexpected (lack of) events"
+        assert META["sha256_16"]["events_" + sc["name"]] == sha16(el.render(*sc["graph"])), \
+            sc["name"] + ": graph changed: re-run tests/golden/make_ref_fixtures.py"
+        got, want = event_log(orc.PortRuntime, sc), META["events"][sc["name"]]
+        assert len(got) == len(want) and all(b0 == b1 and same_as_fingerprint(e0, e1) for (b0, e0), (b1, e1) in zip(got, want)), sc["name"]
+        assert any(ev for _, ev in want) != bool(sc.get("silent")), sc["name"] + ": unexpected (lack of) events"

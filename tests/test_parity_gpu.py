@@ -10,7 +10,8 @@ import numpy as np
 import pytest
 
 from elementary_b200 import Runtime, el, graphs
-from helpers import block_peak_tolerance_check, oracle_render
+from cases import plugin_nodes_batch, plugin_nodes_inputs
+from helpers import block_peak_tolerance_check, oracle_render, reference_extra, sha16
 
 pytestmark = pytest.mark.gpu
 
@@ -546,25 +547,24 @@ def test_control_thread_edits_while_render_thread_processes(tmp_path):
 def test_registered_device_node_types_match_the_reference_plugin_nodes(tile_width):
     """Runtime::registerNodeType (Runtime.h:105-106): two node types registered as CUDA text here and as GraphNode subclasses on the
     reference (oracle/ref_driver.cpp, through the reference's own registerNodeType) render the same samples: a stateless one
-    (all lanes) and a stateful one (owner-lane recurrence whose state survives blocks)."""
-    from oracle import oracle as orc
-    if not orc.ref_available():
-        pytest.skip("needs the compiled reference (its plug-in interface is what is being mirrored)")
+    (all lanes) and a stateful one (owner-lane recurrence whose state survives blocks).  The reference's samples are stored in
+    tests/golden/reference_extra.npz: 64 fixed positions of every block of every voice, and the exact block peaks."""
+    gold, meta = reference_extra()
     n_voices = 5 if tile_width != 32 else 37
-    soft = el.create_node("b200test.softclip", {}, [el.mul(3.0, IN0)])
-    g = el.add(el.create_node("b200test.leaky", {}, [soft, el.const(0.9, key="g")]), el.mul(0.1, el.cycle(330.0)))
-    batch = el.render(g)
+    batch = plugin_nodes_batch()
+    assert meta["sha256_16"]["plugin_nodes"] == sha16(batch), "graph changed: re-run tests/golden/make_ref_fixtures.py"
     opts = {"tile_width": tile_width} if tile_width else {}
     rt = Runtime(SR, BS, n_voices, device=0, **opts)
     assert rt.register_node_type("b200test.softclip", 1, 0, "const float x = in[0]; return x / (1.0f + fabsf(x));") == 0
     assert rt.register_node_type("b200test.leaky", 2, 1, "s[0] = in[0] + in[1] * s[0]; return s[0];") == 0
     assert rt.apply_instructions(batch) == 0, rt.last_error()
-    inputs = np.stack([np.stack([lcg_noise(4 * BS, 100 * v)]) for v in range(n_voices)])
-    got, mix = rt.render_voices(4, 1, inputs)
+    got, mix = rt.render_voices(4, 1, plugin_nodes_inputs(n_voices))
     assert rt.describe()["groups"][0]["spec_state"] == 2
-    ref = oracle_render(batch, 4, 1, SR, BS, inputs, voice_batches=[None] * n_voices, cls=orc.RefRuntime)
-    ok, worst, ex = block_peak_tolerance_check(got, ref, BS)
-    assert ok, f"worst err/tol {worst:.3g}, bit-exact {ex:.4f}"
+    idx = gold["plugin_nodes_idx"]
+    want = gold["plugin_nodes"][:n_voices].astype(np.float64)
+    tol = 1e-5 * gold["plugin_nodes_peak"][:n_voices][..., idx // BS].astype(np.float64) + 1e-7
+    ratio = np.abs(got[..., idx] - want) / tol
+    assert ratio.max() <= 1.0, f"worst err/tol {ratio.max():.3g}, bit-exact {(got[..., idx] == want).mean():.4f}"
 
 
 def test_binary_batch_and_const_table_render_like_the_json_path():
