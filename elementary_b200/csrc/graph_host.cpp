@@ -235,6 +235,7 @@ int Engine::setOption(const char* key, double value) {
     else if (k == "specialize_max_words") { opt_.specializeMaxWords = (int) value; }
     else if (k == "specialize_strict") { opt_.specializeStrict = value != 0; }
     else if (k == "spec_minblocks") { opt_.specMinBlocks = (int) value; }
+    else if (k == "k1_prefetch") { opt_.k1Prefetch = value != 0; }
     else if (k == "time_kernels") { timeKernels_ = value != 0 && !planOnly_; }
     else if (k == "fuse_conv_root") { opt_.fuseConvRoot = value != 0; }
     else if (k == "pipeline_stages") { opt_.pipelineStages = std::max(0, std::min((int) value, (int) MAX_PIPE)); }
@@ -257,6 +258,7 @@ std::string Engine::describe() const {
         if (g->pending || g->active) {
             auto& p = g->pending ? g->pending : g->active;
             os << ",\"slots\":" << p->nSlots << ",\"state_rows\":" << p->nStateRows << ",\"params\":" << p->paramMap.size() << ",\"ops\":" << p->nOps << ",\"code_words\":" << p->code.size()
+               << ",\"promote_at\":" << (p->stages.empty() ? -1 : p->stages.back().promoteAt)
                << ",\"roots\":" << p->rootIds.size() << ",\"pipeline_stages\":" << p->pipeW;
             if (p->specJob) {
                 const int st = p->specJob->state.load(std::memory_order_acquire);
@@ -2122,6 +2124,12 @@ int Engine::compile(Group& g, int nIn, std::shared_ptr<Program>& out) {
     }
     prog->nStateRows = (nStateRows + 1) & ~1;
     prog->nSlots = nSlotsMax;
+    for (auto& st : prog->stages) {   // K1's tap promotion records: directly behind the stage's first OP_END, if there are any
+        size_t pc = st.codeOffset;
+        while (pc < prog->code.size() && (prog->code[pc] & 0xFF) != OP_END) pc += OP_HEADER_WORDS + ((prog->code[pc] >> 8) & 0xFF);
+        pc += OP_HEADER_WORDS;
+        st.promoteAt = (pc < prog->code.size() && (prog->code[pc] & 0xFF) == OP_PROMOTE) ? (int) (pc - st.codeOffset) : -1;
+    }
 
     // ---- upload: code, stateMap and paramMap in ONE allocation; the copies are stream-ordered in front of the first launch and their
     // sources are members of the Program, so nothing has to be waited for here ----
@@ -2332,6 +2340,7 @@ int Engine::enqueueBlock(size_t nIn, size_t nOut, size_t numSamples, bool perVoi
         P.sampleTime = sampleTime_;
         P.tableSrc = p.stagedTable; P.tableFloats = p.stagedTableFloats; P.tableSmem = -1;   // the launcher places it (single-group launches)
         P.pipeW = p.pipeW; P.pipeRingBase = p.pipeRingBase; P.pipeDepth = p.pipeDepth;
+        P.k1Prefetch = opt_.k1Prefetch ? 1 : 0;
         for (int w = 0; w < MAX_PIPE; ++w) { P.pipeCode[w] = p.pipeCode[w]; P.pipeSrow[w] = p.pipeSrow[w]; }
         for (int w = 0; w <= MAX_PIPE; ++w) P.pipeState[w] = p.pipeState[w];
         for (size_t di = 0; di < p.dynNodes.size(); ++di) {
@@ -2369,6 +2378,7 @@ int Engine::enqueueBlock(size_t nIn, size_t nOut, size_t numSamples, bool perVoi
         if (nStages == 1 && groups_.size() > 1 && opt_.batchGroups && !p.hasCustom) {
             // heterogeneous voice groups: collect single-stage groups per tile geometry and launch each bucket once
             P.code = p.dCode + (p.stages.empty() ? 0 : p.stages[0].codeOffset);
+            P.promoteAt = p.stages.empty() ? -1 : p.stages[0].promoteAt;
             // one-voice groups launch through the pipeline kernel (programs that were not cut simply use warp 0 of their CTA): one
             // launch for all of them whether or not every program could be cut
             const int bkey = g.tileWidth + ((p.pipeW > 1 || (g.tileWidth == 1 && opt_.pipelineStages > 1)) ? PIPE_BUCKET : 0);
@@ -2379,6 +2389,7 @@ int Engine::enqueueBlock(size_t nIn, size_t nOut, size_t numSamples, bool perVoi
             allBatched = false;
             const bool last = stg + 1 == nStages;
             P.code = p.dCode + (p.stages.empty() ? 0 : p.stages[stg].codeOffset);
+            P.promoteAt = p.stages.empty() ? -1 : p.stages[stg].promoteAt;
             P.outVoice = (last && materialise) ? voiceOut + (offlineOut_ ? offlineOffset_ : 0) : nullptr;   // outputs and taps belong to the last stage
             P.mixPartial = (last && mix) ? dPartial_ : nullptr;
             std::pair<cudaEvent_t, cudaEvent_t> ev{nullptr, nullptr};

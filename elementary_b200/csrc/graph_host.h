@@ -133,7 +133,8 @@ struct Program {
     unsigned short pipeState[MAX_PIPE + 1] = {0, 0, 0, 0, 0}, pipeSrow[MAX_PIPE] = {0, 0, 0, 0};
     // K1 stages: stage k interprets code[stages[k].codeOffset ...]; after it the convolvers of that stage run (K3)
     struct Conv { int32_t node; float* in; float* out; int inChannel; };   // inChannel >= 0: K3 reads host input channel inChannel directly (no staging copy)
-    struct Stage { uint32_t codeOffset = 0; std::vector<Conv> convolves; bool empty = false; };   // empty: no K1 work in this stage
+    struct Stage { uint32_t codeOffset = 0; std::vector<Conv> convolves; bool empty = false;   // empty: no K1 work in this stage
+                   int promoteAt = -1; };   // LaunchParams::promoteAt of the stage's launch (relative to codeOffset)
     std::vector<Stage> stages;
     // `convolve -> root`: the last stage would only reload the convolver's output and apply the root — K3 does that in its epilogue
     // (convolve.h ConvEpilogue) and the stage's K1 launch is skipped.  fusedConvStage < 0: not fused.
@@ -181,6 +182,7 @@ struct EngineOptions {
                                   // of resident warps, so the gain is far from the stage count (DESIGN.md section 4)
     int specMinBlocks = 0;        // > 0: specialised kernels of the narrow geometries (1 < L < 32) are compiled for this many CTAs per SM (8 = 64 registers)
     bool specializeStrict = false; // a failed specialisation is an error (COMMIT returns 7 / process -1) instead of a silent stay on the interpreter
+    bool k1Prefetch = true;       // LaunchParams::k1Prefetch: false forces K1's plain paths (the bit-identical reference of tests and A/B runs)
 };
 
 class Engine {

@@ -160,6 +160,12 @@ struct LaunchParams {
     uint32_t pipeCode[MAX_PIPE];            // word offset of stage w's code behind `code`
     unsigned short pipeState[MAX_PIPE + 1]; // stage w owns stateMap entries [pipeState[w], pipeState[w + 1])
     unsigned short pipeSrow[MAX_PIPE];      // first shared-memory state row of stage w
+    int promoteAt;               // word offset of the first OP_PROMOTE record behind `code`, -1 = the program has none
+    // Engine option "k1_prefetch" (default 1).  The kernel chooses its latency-hiding paths (prologue rows staged by cp.async outside
+    // the one-voice pipeline kernel, delay ring reads of a tile issued together, no program walk to find the tap promotion records) from what it sees: parameter-row delay
+    // lengths and their distance from the tile's writes.  0 forces the plain paths those fall back to; it is a reference for tests
+    // and A/B runs, not a tuning knob — both compute the same bits.
+    int k1Prefetch;
 };
 constexpr int TABLE_SMEM_MAX_FLOATS = 8192;   // tables up to 32 KB are staged
 

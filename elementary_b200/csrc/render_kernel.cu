@@ -58,6 +58,10 @@ struct SP {
 
 // ---- TMA (1-D bulk async copy) + mbarrier: stages a program's wavetable HBM -> shared memory once per CTA (SASS: UBLKCP)
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t) __cvta_generic_to_shared(p); }
+// ---- cp.async (LDGSTS): global -> shared copies that do not hold up the issuing warp; completed by cp.async.wait_all
+__device__ __forceinline__ void cp_async_4(uint32_t dst, const void* src) { asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory"); }
+__device__ __forceinline__ void cp_async_8(uint32_t dst, const void* src) { asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(dst), "l"(src) : "memory"); }
+
 __device__ __forceinline__ void stage_table_tma(const float* src, int floats, float* dst, uint64_t* bar) {
     if (threadIdx.x == 0) {
         asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(bar)) : "memory");
@@ -553,7 +557,37 @@ __device__ __forceinline__ void render_tile(const LaunchParams& P, const int til
     const int stateBegin = (PIPE && pipeW > 1) ? (int) P.pipeState[stage] : 0;
     const int stateEnd = (PIPE && pipeW > 1) ? (int) P.pipeState[stage + 1] : P.nStateEntries;
     const int srowBegin = (PIPE && pipeW > 1) ? (int) P.pipeSrow[stage] : 0;
-    if (owner) {
+    if (!PIPE && P.k1Prefetch) {
+        // Two dependent round trips in all: every lane loads one map entry, then the owner lanes issue all row copies back to back
+        // as cp.async (LDGSTS) and wait once.  (A load-then-store loop waits for each row before it issues the next map load: with
+        // the L2 cold that is some twenty HBM round trips per warp before the first sample.)  The one-voice pipeline kernel keeps the
+        // plain loop: there this code costs spill loads inside the 64-register interpreter loop (BASELINE config 5 ran 5 % slower).
+        const int nSt = stateEnd - stateBegin, nPar = firstStage ? P.nParams : 0;
+        int srow = srowBegin;
+        for (int c0 = 0; c0 < max(nSt, nPar); c0 += 32) {
+            const uint32_t ms = (c0 + lane < nSt) ? __ldg(P.stateMap + stateBegin + c0 + lane) : STATE_PAD;
+            const uint32_t mp = (c0 + lane < nPar) ? __ldg(P.paramMap + c0 + lane) : 0u;
+            for (int j = 0, jn = min(32, nSt - c0); j < jn; ++j) {
+                const uint32_t m = __shfl_sync(FULL, ms, j);
+                if (m == STATE_PAD) { srow += 1; continue; }
+                const size_t row = m & ~STATE_DOUBLE_FLAG;
+                if (m & STATE_DOUBLE_FLAG) {
+                    if (owner) cp_async_8(smem_u32(reinterpret_cast<double*>((sst + srow * L).ptr()) + lane),
+                                          reinterpret_cast<const double*>(P.rows + row * P.Vpad) + voice);
+                    srow += 2;
+                } else {
+                    if (owner) cp_async_4(smem_u32((sst + (srow * L + lane)).ptr()), P.rows + row * P.Vpad + voice);
+                    srow += 1;
+                }
+            }
+            for (int j = 0, jn = min(32, nPar - c0); j < jn; ++j) {
+                const uint32_t m = __shfl_sync(FULL, mp, j);
+                if (owner) cp_async_4(smem_u32((spar + ((c0 + j + 1) * L + lane)).ptr()), P.rows + (size_t) m * P.Vpad + voice);
+            }
+        }
+        if (firstStage && owner) spar[lane] = 0.0f;
+        asm volatile("cp.async.wait_all;" ::: "memory");
+    } else if (owner) {
         int srow = srowBegin;
         for (int i = stateBegin; i < stateEnd; ++i) {
             const uint32_t m = __ldg(P.stateMap + i);
@@ -818,9 +852,11 @@ __device__ __forceinline__ void render_tile(const LaunchParams& P, const int til
     }
 
     // ---- tap promotion (GraphRenderSequence.h:200-210,306-308): OP_PROMOTE records after the first OP_END ----
-    if (!(PIPE && pipeW > 1)) {    // (the host never pipelines a program with taps)
+    // (the host never pipelines a program with taps; it also knows where the records start, so most programs skip this entirely)
+    if (!(PIPE && pipeW > 1) && (!P.k1Prefetch || P.promoteAt >= 0)) {
         const uint32_t* pc = P.code;
-        for (;;) {   // skip the main program
+        if (P.k1Prefetch) pc += P.promoteAt;
+        else for (;;) {   // skip the main program
             const uint32_t w0 = __ldg(pc);
             pc += OP_HEADER_WORDS + ((w0 >> 8) & 0xFF);
             if ((w0 & 0xFF) == OP_END) break;
